@@ -9,6 +9,7 @@ attention readout, 2-layer MLP head, BCE loss, backward, gradient all-reduce (N>
 data-path collective).
 
   python bench.py --gpus 1 --steps K --warmup W            # our arm (CUDA, libddfa_b200.so)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # ... and the last timed step's loss + parameters as .npy
   python bench.py --impl reference --steps K --warmup W    # reference arm: the reference path's CPU
                                                            # restatement (oracle/) on the host cores
 One JSON line on stdout (rank 0).  See DESIGN.md §6 for every field.
@@ -35,7 +36,6 @@ CFG = dict(graphs=1024, nodes=150, edges_per_node=2.0, input_dim=1002, hidden_di
 METRIC = "CFG graphs/sec (train step)"
 UNIT = "graphs/s"
 NUM_BATCHES = 8  # distinct resident batches rotated through the timed region
-MIN_TIMED_MS = float(os.environ.get("DDFA_BENCH_MIN_TIMED_MS", "300"))  # (0 for profiler runs) the K-step timed region is repeated until this much device time is covered; the median region is reported
 
 
 def workload_tag(graphs):
@@ -226,7 +226,9 @@ def run_reference(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if rank != 0:
         return 0
-    val, s_per_step, done, threads = cpu_train_steps(args.graphs, args.steps, max(min(args.warmup, 2), 1), budget_s=180.0)
+    if args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs writes the CUDA arm's outputs; it has no --impl reference form")
+    val, s_per_step, done, threads = cpu_train_steps(args.graphs, args.steps, max(min(args.warmup, 2), 1))
     out = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": done, "warmup": args.warmup,
         "ms_per_step": s_per_step * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -258,26 +260,31 @@ class Ctx:
     pass
 
 
-def timed_regions(ctx, fn_step, steps, min_ms=MIN_TIMED_MS, max_regions=25):
-    """Times regions of EXACTLY `steps` steps each (barrier + synchronize on both sides, CUDA events, max over ranks) until
-    `min_ms` of device time is covered; returns the per-region milliseconds."""
+def timed_steps(ctx, fn_step, steps):
+    """Milliseconds of EXACTLY `steps` calls of fn_step (barrier + synchronize on both sides, CUDA events, max over ranks)."""
     import torch.distributed as dist
-    out = []
-    while True:
-        ctx.barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for i in range(steps):
-            fn_step(i)
-        e1.record()
-        ctx.barrier()
-        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=ctx.dev)
-        if ctx.world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        out.append(float(t.item()))
-        # every rank sees the same (max-reduced) numbers, so all ranks leave the loop together
-        if sum(out) >= min_ms or len(out) >= max_regions:
-            return out
+    ctx.barrier()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for i in range(steps):
+        fn_step(i)
+    e1.record()
+    ctx.barrier()
+    t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=ctx.dev)
+    if ctx.world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return float(t.item())
+
+
+def dump_outputs(trainer, out_dir):
+    """Writes what the caller of the timed step holds after the last timed step — the loss it returned and the module's updated
+    parameters — as float32 <out_dir>/<name>.npy (1.2 MB at the default sizes), so two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": trainer.loss_slot}
+    arrays.update({f"param.{k}": p for k, p in trainer.module.named_parameters()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def roofline_lines(prof, ms_region, N, Eg, engine, peaks, mode_tag):
@@ -410,7 +417,7 @@ def measure_workload(ctx, args, graphs, full):
             graph_note = f"off (capture failed: {type(exc).__name__}: {str(exc)[:120]})"
     res["cuda_graph"] = graph_note
 
-    # ---- timed regions (headline): K resident-input train steps each ----------------------------------------------------
+    # ---- timed region (headline): K resident-input train steps -------------------------------------------------------------
     sampler = ClockSampler(ctx.local_rank)
     if rank == 0 and full:
         sampler.start()
@@ -418,15 +425,16 @@ def measure_workload(ctx, args, graphs, full):
     for i in range(warm):
         step_dev(i)
     t_wall0 = time.time()
-    regions = timed_regions(ctx, step_dev, steps)
+    ms_total = timed_steps(ctx, step_dev, steps)
     t_wall1 = time.time()
-    ms_total = statistics.median(regions)
     if rank == 0 and full:
         res["clocks"] = sampler.stop(t_wall0, t_wall1)
+        if args.dump_outputs:
+            dump_outputs(trainer, args.dump_outputs)
     res["final_loss"] = float(trainer.loss_slot.item())
     res["value"] = global_batch * steps / (ms_total * 1e-3)
     res["ms_per_step"] = ms_total / steps
-    res["timed_regions"] = {"count": len(regions), "steps_each": steps, "ms": [round(x, 3) for x in regions], "reported": "median"}
+    res["timed_ms"] = round(ms_total, 3)
     res["gpu_launches_per_step"] = int(launches_per_step)
     res["nodes"], res["edges"] = N, Eg
 
@@ -444,10 +452,9 @@ def measure_workload(ctx, args, graphs, full):
         state["nxt"] = fresh(host_batches[(i + 1) % NUM_BATCHES])
         trainer.prefetch(state["nxt"], global_batch)          # the next step's H2D copies run on a side stream during this step
         state["loss"] = float(loss_t.item())
-    e2e_regions = timed_regions(ctx, step_e2e, steps, min_ms=MIN_TIMED_MS / 2, max_regions=10)
-    ms_e2e = statistics.median(e2e_regions)
+    ms_e2e = timed_steps(ctx, step_e2e, steps)
     res["e2e"] = {"value": global_batch * steps / (ms_e2e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": batch_bytes(host_batches[0]),
-                  "d2h_bytes_per_step": 4, "steps": steps, "regions": len(e2e_regions),
+                  "d2h_bytes_per_step": 4, "steps": steps,
                   "path": "FusedTrainer.step(host batch): pinned host COO + node indices -> H2D -> ddfa_build_csr -> fused train step -> loss .item()"
                           + (" (one CUDA graph per batch shape, two static input-buffer sets, next batch prefetched on a copy stream)"
                              if trainer.use_cuda_graph else " (eager launches)")}
@@ -465,8 +472,8 @@ def measure_workload(ctx, args, graphs, full):
 
     def step_arena(i):
         state["loss"] = float(trainer.step_ids(arena, id_lists[i % NUM_BATCHES], global_batch).item())
-    ar_regions = timed_regions(ctx, step_arena, steps, min_ms=MIN_TIMED_MS / 2, max_regions=10)
-    res["e2e_arena"] = {"value": global_batch * steps / (statistics.median(ar_regions) * 1e-3), "unit": UNIT, "h2d_bytes_per_step": 4 * graphs,
+    ms_arena = timed_steps(ctx, step_arena, steps)
+    res["e2e_arena"] = {"value": global_batch * steps / (ms_arena * 1e-3), "unit": UNIT, "h2d_bytes_per_step": 4 * graphs,
                         "d2h_bytes_per_step": 4, "steps": steps,
                         "path": f"graph-id list (pinned) -> H2D -> ddfa_arena_batch over a resident arena of {arena.num_graphs} graphs -> "
                                 "fused train step -> loss .item()", "last_loss": state["loss"]}
@@ -488,8 +495,8 @@ def measure_workload(ctx, args, graphs, full):
             state["loss"] = float(loss.item())
         for i in range(3):
             step_api(i)
-        api_regions = timed_regions(ctx, step_api, steps, min_ms=MIN_TIMED_MS / 2, max_regions=10)
-        res["e2e_module_api"] = {"value": global_batch * steps / (statistics.median(api_regions) * 1e-3), "unit": UNIT,
+        ms_api = timed_steps(ctx, step_api, steps)
+        res["e2e_module_api"] = {"value": global_batch * steps / (ms_api * 1e-3), "unit": UNIT,
                                  "h2d_bytes_per_step": batch_bytes(host_batches[0]), "d2h_bytes_per_step": 4, "steps": steps,
                                  "path": "FlowGNNGGNNModule.training_step((host batch, {})) -> loss.backward() -> torch.optim.Adam.step() -> "
                                          "loss.item()  (autograd Function around the same kernels, eager launches, per-step allocation)",
@@ -528,10 +535,9 @@ def measure_variable_stream(ctx, args, graphs):
         state["nxt"] = fresh(host[(i + 1) % n_batches])
         trainer.prefetch(state["nxt"], global_batch)
         state["loss"] = float(loss_t.item())
-    regions = timed_regions(ctx, step_var, n_batches, min_ms=MIN_TIMED_MS / 2, max_regions=6)
-    ms = statistics.median(regions)
+    ms = timed_steps(ctx, step_var, args.steps)
     shapes = sorted({(b.num_nodes(), b.num_edges()) for b in host})
-    return {"value": global_batch * n_batches / (ms * 1e-3), "unit": UNIT, "ms_per_step": ms / n_batches, "steps": n_batches,
+    return {"value": global_batch * args.steps / (ms * 1e-3), "unit": UNIT, "ms_per_step": ms / args.steps, "steps": args.steps,
             "distinct_batch_shapes": len(shapes), "mean_nodes_per_batch": nodes, "bucket_shapes_captured": trainer.num_bucket_shapes(),
             "path": "FusedTrainer.step(host batch), variable=True lognormal graph sizes (mean 150 nodes), every batch a new (N, E); padded to bucket "
                     "shapes (one dummy graph of isolated nodes, zero loss weight), one CUDA graph per bucket shape, next batch prefetched; loss .item() every step",
@@ -584,7 +590,7 @@ def run_ours(args):
     if args.secondary and args.graphs == 1024:
         s = measure_workload(ctx, args, 256, full=False)
         secondary.append({"config": workload_config(256, world), "value": s["value"], "unit": UNIT, "ms_per_step": s["ms_per_step"],
-                          "e2e": s["e2e"], "cuda_graph": s["cuda_graph"], "timed_regions": s["timed_regions"]})
+                          "e2e": s["e2e"], "cuda_graph": s["cuda_graph"], "timed_ms": s["timed_ms"]})
     variable = measure_variable_stream(ctx, args, args.graphs) if args.variable else None
 
     def leave():
@@ -617,7 +623,7 @@ def run_ours(args):
         "data": "synthetic", "config": workload_config(args.graphs, world),
         "engine": args.engine,
         "l2": f"per-step working set ~{N * 128 * 4 * 49 / 1e9:.2f} GB of saved activations > 126 MB L2; {NUM_BATCHES} distinct resident batches rotated",
-        "timed_regions": primary["timed_regions"],
+        "timed_ms": primary["timed_ms"],
         "clocks": primary.get("clocks"),
         "e2e": primary["e2e"], "e2e_arena": primary.get("e2e_arena"), "e2e_module_api": primary.get("e2e_module_api"),
         "e2e_variable": variable,
@@ -650,6 +656,8 @@ def main():
     ap.add_argument("--no-secondary", dest="secondary", action="store_false", help="skip the C0 second workload of the default run")
     ap.add_argument("--no-variable", dest="variable", action="store_false", help="skip the variable-shape stream line")
     ap.add_argument("--quick", action="store_true", help="headline value + e2e only (no per-kernel spans, arena / module-API lines, CPU baseline): scaling A/Bs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the loss and the updated parameters of the last one "
+                                                          "to DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

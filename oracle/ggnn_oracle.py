@@ -17,7 +17,7 @@ PARITY STATUS: **partially pinned**.
     ``BaseModule.__init__ / get_label / training_step`` (base_module.py:27-95, 171-199) — has been EXECUTED in the build
     container with stand-ins for its bookkeeping imports (Lightning, torchmetrics, deepspeed, nni) and with the two DGL
     operators bound to the restatements below (``tests/golden/make_reference_ctrlflow_golden.py``); its outputs, labels,
-    training loss, gradients and state_dict are committed (``tests/golden/reference_ctrlflow_golden.pt``) and
+    training loss, gradients (the larger ones sampled) and state_dict are committed (``tests/golden/reference_ctrlflow_golden.pt.xz``) and
     ``tests/test_oracle.py::test_oracle_matches_reference_control_flow`` pins this oracle against them.  So parameter
     construction and naming, embedding order, concatenations, pooling / MLP placement, ``squeeze``, ``encoder_mode``, the
     graph-label rule and the loss are pinned to the reference's executing code.

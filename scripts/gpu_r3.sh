@@ -6,7 +6,7 @@ set -u
 TAG=$1; shift
 OUT=gpurun_out
 mkdir -p $OUT
-PROF_ENV="DDFA_BENCH_MIN_WARMUP=1 DDFA_BENCH_SKIP_CPU=1 DDFA_BENCH_MIN_TIMED_MS=0"
+PROF_ENV="DDFA_BENCH_MIN_WARMUP=1 DDFA_BENCH_SKIP_CPU=1"
 for STAGE in "$@"; do
   echo "=================== stage: $STAGE"
   case $STAGE in

@@ -14,8 +14,11 @@ fixture therefore pins, against the reference's own executing code: parameter co
 feature-key and embedding order, the concatenations, where pooling and the MLP sit, `.squeeze()`, `encoder_mode`, the
 graph-label rule (`dgl.unbatch` + max of `_VULN`), `BCEWithLogitsLoss(pos_weight)` and the training-step loss.
 
-Run in the build container (needs /root/reference):   python tests/golden/make_reference_ctrlflow_golden.py
-Writes tests/golden/reference_ctrlflow_golden.pt; tests/test_oracle.py::test_oracle_matches_reference_control_flow reads it.
+The parameters are set from tests/golden_params.py's hash before the reference code runs, so the fixture stores their names,
+shapes and bounds instead of their values, and a sample of each large gradient (see that module).
+
+Run with a checkout of ISU-PAAL/DeepDFA:   python tests/golden/make_reference_ctrlflow_golden.py <DeepDFA>/DDFA
+Writes tests/golden/reference_ctrlflow_golden.pt.xz; tests/test_oracle.py::test_oracle_matches_reference_control_flow reads it.
 """
 import inspect
 import os
@@ -27,8 +30,9 @@ from torch import nn
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-REFERENCE = "/root/reference/DDFA"
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+from golden_params import hash_params, sample, save, stored_state  # noqa: E402
 from deepdfa_b200 import batched_graph as BG  # noqa: E402
 from deepdfa_b200 import synth  # noqa: E402
 from oracle import ggnn_oracle as O  # noqa: E402
@@ -111,9 +115,9 @@ def install_stand_ins():
     sys.modules.update(mods)
 
 
-def main():
+def main(reference):
     install_stand_ins()
-    sys.path.insert(0, REFERENCE)
+    sys.path.insert(0, reference)
     from code_gnn.models.flow_gnn.ggnn import FlowGNNGGNNModule as RefModule      # the real reference class
 
     feat = "_ABS_DATAFLOW_datatype_all_limitall_1000_limitsubkeys_1000"
@@ -148,10 +152,11 @@ def main():
         ref = RefModule(**spec["ctor"])
         with torch.no_grad():
             ref.ggnn.linears[0].bias.uniform_(-0.1, 0.1)             # DGL zero-initialises it; make the bias path visible
+        params = hash_params(ref, 100 + i)
         g = synth.make_batch(**spec["graphs"])
         if not spec["ctor"].get("concat_all_absdf"):
             g.ndata["_ABS_DATAFLOW"] = g.ndata["_ABS_DATAFLOW_datatype"] % spec["ctor"]["input_dim"]
-        case = {"name": spec["name"], "ctor": spec["ctor"], "state_dict": {k: v.clone() for k, v in ref.state_dict().items()},
+        case = {"name": spec["name"], "ctor": spec["ctor"], "state_dict": stored_state(ref, params), "params": params,
                 "graph": {"src": g.edges()[0], "dst": g.edges()[1], "batch_num_nodes": g.batch_num_nodes(), "ndata": dict(g.ndata)}}
         ref.eval()
         with torch.no_grad():
@@ -165,12 +170,12 @@ def main():
             loss = ref.training_step((g, {}), 0)
             loss.backward()
             case["train_loss"] = loss.detach().clone()
-            case["grads"] = {k: p.grad.clone() for k, p in ref.named_parameters() if p.grad is not None}
+            case["grads"] = {k: sample(p.grad, 100 * i + j) for j, (k, p) in enumerate(ref.named_parameters()) if p.grad is not None}
         cases.append(case)
-    out = os.path.join(ROOT, "tests", "golden", "reference_ctrlflow_golden.pt")
-    torch.save({"cases": cases, "note": "outputs of the reference's own ggnn.py / base_module.py code; DGL ops bound to the oracle restatements"}, out)
+    out = save({"cases": cases, "note": "outputs of the reference's own ggnn.py / base_module.py code; DGL ops bound to the oracle restatements"},
+               "reference_ctrlflow_golden.pt.xz")
     print("wrote", out, {c["name"]: tuple(c["out"].shape) for c in cases})
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

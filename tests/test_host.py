@@ -154,9 +154,9 @@ def test_analytic_counts_and_count_strings():
 
 def test_module_state_dict_matches_the_reference_classes():
     """Key names and shapes of FlowGNNGGNNModule.state_dict() vs the state_dict the REAL reference classes produced
-    (tests/golden/reference_ctrlflow_golden.pt, written by make_reference_ctrlflow_golden.py), incl. loss_fn.pos_weight."""
-    import os
-    data = torch.load(os.path.join(os.path.dirname(__file__), "golden", "reference_ctrlflow_golden.pt"), weights_only=False)
+    (tests/golden/reference_ctrlflow_golden.pt.xz, written by make_reference_ctrlflow_golden.py), incl. loss_fn.pos_weight."""
+    from golden_params import load
+    data = load("reference_ctrlflow_golden.pt.xz")
     for case in data["cases"]:
         m = D.FlowGNNGGNNModule(**case["ctor"])
         ours, ref = m.state_dict(), case["state_dict"]

@@ -1,7 +1,6 @@
 """LineVul + DeepDFA combined head (SURVEY.md §8 f3, BASELINE configs[4]): ``deepdfa_b200.linevul.LineVulCombined`` against
 outputs of the reference's own ``linevul_model.Model`` (tests/golden/make_reference_linevul_golden.py), and the eval harness
 of ``linevul_main.evaluate`` (F1 at the 0.5 threshold) with the CUDA encoder against the oracle encoder under one frozen head."""
-import os
 import time
 
 import numpy as np
@@ -11,9 +10,10 @@ import torch
 from deepdfa_b200 import synth
 from deepdfa_b200.batched_graph import BatchedCFG
 from deepdfa_b200.linevul import LineVulCombined, evaluate
+from golden_params import load
 from oracle import ggnn_oracle as O
 
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference_linevul_golden.pt")
+GOLDEN = "reference_linevul_golden.pt.xz"
 DEV = "cuda:0"
 
 
@@ -37,7 +37,7 @@ def _graph(data):
 def test_wrapper_reproduces_reference_model_on_cpu():
     """Control flow, head and state_dict naming of the wrapper are the reference's: with the oracle as flowgnn_encoder (what the
     fixture was generated with) the outputs are identical."""
-    data = torch.load(GOLDEN, weights_only=False)
+    data = load(GOLDEN)
     model = _build(data, O.OracleFlowGNNGGNN(**data["flow"]))
     g = _graph(data)
     with torch.no_grad():
@@ -53,7 +53,7 @@ def test_wrapper_reproduces_reference_model_on_cpu():
 @pytest.mark.parametrize("engine", ["simt", "tcgen05"])
 def test_cuda_encoder_under_the_reference_head(engine):
     import deepdfa_b200 as D
-    data = torch.load(GOLDEN, weights_only=False)
+    data = load(GOLDEN)
     flow = D.FlowGNNGGNNModule(**data["flow"], engine=engine)
     model = _build(data, flow, DEV)
     g = _graph(data)
@@ -74,7 +74,7 @@ def test_eval_f1_gpu_encoder_vs_oracle_encoder_and_stream_overlap():
     encoder on the CPU and (b) the CUDA encoder — with and without the side-stream overlap."""
     import deepdfa_b200 as D
     learnable_batch = synth.make_learnable_batch
-    data = torch.load(GOLDEN, weights_only=False)
+    data = load(GOLDEN)
     torch.manual_seed(1)
     oracle_flow = O.OracleFlowGNNGGNN(**data["flow"])
     cpu_model = _build(data, oracle_flow)

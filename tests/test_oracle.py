@@ -105,7 +105,10 @@ def test_golden_vectors(golden):
         g = graph_of(case)
         with torch.no_grad():
             out32 = m32(g)
-        assert torch.equal(out32, case["out_fp32"]), case["name"]
+        # fp32 on another CPU runs other kernels (vector width, summation order), so only the last bits are free: 64 ulps of
+        # the output's scale (other instruction sets measured up to 14); the fp64 pin below stays at 1e-12
+        ulp = torch.finfo(torch.float32).eps * float(case["out_fp32"].abs().max())
+        assert (out32 - case["out_fp32"]).abs().max() <= 64 * ulp, case["name"]
         m64 = build(case, torch.float64)
         m64.load_state_dict({k: v.double() for k, v in sd.items()})
         with torch.no_grad():
@@ -197,10 +200,9 @@ def test_oracle_matches_reference_control_flow():
     real FlowGNNGGNNModule + BaseModule with stand-ins for the bookkeeping imports; the two DGL operators bound to the oracle's
     restatements).  It pins the oracle's — and therefore the module's — restatement of that code: parameter names and shapes,
     embedding order, concatenations, pooling / MLP placement, squeeze, encoder_mode, graph labels, BCE(pos_weight), gradients."""
-    import os
     from deepdfa_b200.batched_graph import BatchedCFG
-    path = os.path.join(os.path.dirname(__file__), "golden", "reference_ctrlflow_golden.pt")
-    data = torch.load(path, weights_only=False)
+    from golden_params import load, sample_error
+    data = load("reference_ctrlflow_golden.pt.xz")
     assert len(data["cases"]) == 8 and sum(c["ctor"].get("label_style") == "node" for c in data["cases"]) == 2 and any("grads" in c and c["ctor"]["hidden_dim"] == 32 for c in data["cases"])
     for case in data["cases"]:
         gd = case["graph"]
@@ -225,5 +227,6 @@ def test_oracle_matches_reference_control_flow():
             assert torch.allclose(loss, case["train_loss"], atol=1e-6, rtol=1e-5), case["name"]
             grads = {k: p.grad for k, p in o.named_parameters() if p.grad is not None}
             assert set(grads) == set(case["grads"]), case["name"]
-            for k, gref in case["grads"].items():
-                assert torch.allclose(grads[k], gref, atol=1e-6, rtol=1e-4), (case["name"], k)
+            for k, s in case["grads"].items():
+                assert torch.allclose(grads[k].flatten()[s["idx"].long()], s["val"], atol=1e-6, rtol=1e-4), (case["name"], k)
+                assert sample_error(grads[k], s) <= 1e-6 + 1e-4 * s["absmax"], (case["name"], k)
