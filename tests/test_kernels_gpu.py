@@ -8,6 +8,8 @@ from deepdfa_b200 import synth
 from deepdfa_b200._lib import ENGINE_SIMT, ENGINE_TCGEN05, DdfaError, lib, ptr_array
 from deepdfa_b200.engine import _p, _stream_ptr, prepare_graph
 from oracle import ggnn_oracle as O
+from parity_helpers import decode_gates, decode_image
+from parity_helpers import gru_reference as _gru_reference
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -218,15 +220,6 @@ def test_fold_weights_fwd_bwd():
         assert (got.cpu().double() - 1.0 - ref).abs().max() < 1e-3 * max(1.0, float(ref.abs().max()) / 10)
 
 
-def _gru_reference(s, h, deg, wf, bf, bih, whh, bhh):
-    D = h.shape[1]
-    gi = s @ wf.t() + deg[:, None] * bf[None, :] + bih
-    gh = h @ whh.t() + bhh
-    r = torch.sigmoid(gi[:, :D] + gh[:, :D]); z = torch.sigmoid(gi[:, D:2 * D] + gh[:, D:2 * D])
-    n = torch.tanh(gi[:, 2 * D:] + r * gh[:, 2 * D:])
-    return (1 - z) * n + z * h, r, z, n, gh[:, 2 * D:]
-
-
 @pytest.mark.parametrize("D", [32, 128, 256])
 def test_gru_step_fwd_bwd(D):
     g = synth.make_batch(24, 60, seed=2, variable=True)
@@ -357,34 +350,6 @@ def test_gru_step_image_entries(graphs, nodes):
         L.call("ddfa_gru_step_bwd_image", _p(dpart_d), _p(ds), _p(dg.indptr_t), _p(dg.indices_t), _p(hd), _p(h_img), _p(s_img), _p(gates),
                _p(dg.indptr), N, D, _p(ds), _p(dh), _p(acc["dwf"]), _p(acc["dbf"]), _p(acc["dbih"]), _p(acc["dwhh"]), _p(acc["dbhh"]),
                _p(ws_b), wsb_b, 0, st())
-
-
-def decode_image(img: torch.Tensor, N: int) -> torch.Tensor:
-    """Activation image (include/ddfa_b200.h) -> fp64 [N,128] = hi + lo, undoing the SWIZZLE_128B unit permutation."""
-    tiles = img.numel() // 65536
-    raw = img.cpu().view(torch.int16).view(tiles, 4, 128, 8, 8)                   # [tile][chunk = 2 v + kb][row][physical 16-B unit][8 bf16]
-    rows = torch.arange(128).view(1, 1, 128, 1, 1)
-    units = torch.arange(8).view(1, 1, 1, 8, 1)
-    phys = (units ^ (rows & 7)).expand(tiles, 4, 128, 8, 8)
-    logical = torch.gather(raw, 3, phys)                                          # logical unit j sits at physical unit j ^ (row & 7)
-    vals = (logical.to(torch.int32) << 16).view(torch.float32).double().view(tiles, 2, 2, 128, 64)   # [tile][v][kb][row][col in block]
-    x = (vals[:, 0] + vals[:, 1]).permute(0, 2, 1, 3).reshape(tiles * 128, 128)   # hi + lo, [row][kb][64] -> 128 columns
-    assert float(x[N:].abs().max()) == 0.0 if x.shape[0] > N else True           # rows past N are zero
-    return x[:N]
-
-
-def decode_gates(gates: torch.Tensor, N: int):
-    """Packed saved gates (csrc/tc_common.cuh: pack_gates) -> (r, z, n, gh_n) fp64 [N,128]."""
-    w = gates.cpu().view(torch.int32).view(N, 128, 2).to(torch.int64) & 0xffffffff
-    x, y = w[..., 0], w[..., 1]
-    r = (x & 0x3fff).double() / 16383.0
-    z = ((x >> 14) & 0x3fff).double() / 16383.0
-    nq = y & 0xffff
-    n = torch.where(nq >= 32768, nq - 65536, nq).double() / 32767.0
-    g = ((y >> 16) << 4) | (x >> 28)
-    e, m, sign = (g >> 14) & 31, (g & 0x3fff).double(), (g >> 19) & 1
-    ghn = torch.where(e == 0, torch.zeros_like(m), torch.pow(2.0, (e - 15).double()) * (1.0 + m / 16384.0))
-    return r, z, n, torch.where(sign == 1, -ghn, ghn)
 
 
 @pytest.mark.parametrize("graphs,nodes", [(3, 50), (24, 60), (40, 150)])
